@@ -1,6 +1,7 @@
 """Benchmark of the RigL hot path: sparse train step (+ the periodic mask update) on B200.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2|c3|c4|c5] [--impl ours|reference]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Configs (BASELINE.json `configs`; the metric is quoted on c2, the default):
@@ -14,6 +15,7 @@ first one falls in the middle of the region), so `value` includes their cost at 
 or denser.  One JSON line on rank 0: the driver contract plus `roofline`, `cpu_baseline`, `mask_update_ms`.
 """
 import argparse
+import functools
 import json
 import os
 import subprocess
@@ -174,6 +176,41 @@ def masked_flops_per_image(model, image, dev):
           'algorithmic_gflop': (2 * f_s + f_d - first_s) / 1e9, 'dense_executed_gflop': (3 * f_d - first_d) / 1e9}
 
 
+DUMP_SAMPLE = 1 << 21       # elements per dumped array (8 MB in float32): a whole dump stays under 41 MB
+
+
+@functools.lru_cache(maxsize=None)
+def _dump_index(n):
+  """A fixed, seeded sample of DUMP_SAMPLE of the positions 0..n-1, ascending."""
+  return torch.from_numpy(np.sort(np.random.RandomState(0).choice(n, DUMP_SAMPLE, replace=False)))
+
+
+def _dump_sample(t):
+  return t if t.numel() <= DUMP_SAMPLE else t[_dump_index(t.numel()).to(t.device)]
+
+
+def dump_outputs(out_dir, model, harness, loss):
+  """Writes what the last timed step computed as DIR/<name>.npy (float32): its loss and the model it leaves behind.
+  The per-layer arrays are concatenated in registry order (each layer flat, C order) and sampled at the same
+  positions: masked weights, masks, momentum slots and the step's dense gradients; other_params holds every
+  parameter that carries no mask (batch-norm scales and offsets, biases, dense depthwise weights)."""
+  os.makedirs(out_dir, exist_ok=True)
+  layers = model.registry.layers()
+  masked = set(id(l.weight) for l in layers)
+  parts = {
+      'masked_weights': [l.weight.reshape(-1) for l in layers],
+      'masks': [l.mask.to_dense().reshape(-1) for l in layers],
+      'momentum': [harness.inner.state[l.weight]['momentum_buffer'].reshape(-1) for l in layers],
+      'dense_grads': [l.masked_weights.dense_grad.reshape(-1) for l in layers],
+      'other_params': [p.reshape(-1) for p in model.parameters() if id(p) not in masked],
+  }
+  arrays = {'loss': loss.float().reshape(())}
+  for name, ts in parts.items():
+    arrays[name] = _dump_sample(torch.cat([t.detach().float() for t in ts]))
+  for name, t in arrays.items():
+    np.save(os.path.join(out_dir, name + '.npy'), t.cpu().numpy())
+
+
 def run_ours(args):
   from rigl_b200 import _cabi
   from rigl_b200 import workloads
@@ -236,13 +273,16 @@ def run_ours(args):
   marks[0].record()
   n_updates, update_steps = 0, []
   for i in range(args.steps):
-    harness.step(images, labels)
+    loss = harness.step(images, labels).detach()      # (keeps no autograd graph alive into the next step)
     marks[i + 1].record()
     if harness.opt.last_update_was_mask_update:
       n_updates += 1
       update_steps.append(i)
   stop.record()
   barrier()
+  if args.dump_outputs and rank == 0:
+    # before the legs below train on and change the model
+    dump_outputs(args.dump_outputs, model, harness, loss)
   per_step = [marks[i].elapsed_time(marks[i + 1]) for i in range(args.steps)]
   clocks = sampler.stop() if rank == 0 else None
   launches = _cabi.launch_count() + getattr(harness, 'replayed_kernel_launches', 0) - launches0
@@ -515,7 +555,14 @@ def main():
   ap.add_argument('--scaling', default='weak', choices=['weak', 'strong'],
                   help='weak (default, the driver contract): the per-GPU batch is fixed; strong: the GLOBAL batch of '
                        'the config is fixed and split over the ranks')
+  ap.add_argument('--dump-outputs', default=None, metavar='DIR',
+                  help='write what the last timed step computed (loss, sampled weights / masks / momentum / dense '
+                       'gradients, other parameters) as DIR/<name>.npy, to compare two builds on the same inputs')
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl != 'ours':
+    ap.error('--dump-outputs writes the outputs of --impl ours')
   if args.warmup < 3 and args.impl == 'ours':
     args.warmup = 3
   if args.impl == 'reference':

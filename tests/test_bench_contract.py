@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -50,6 +52,24 @@ def test_product_arm_refuses_to_run_without_a_gpu():
   r = _run(['--steps', '1', '--warmup', '0', '--no-cpu-baseline'], timeout=300)
   assert r.returncode != 0, 'bench.py must not fall back to a CPU path'
   assert r.stdout.strip() == '', 'and must not print a bench line'
+
+
+@pytest.mark.gpu
+def test_product_arm_dumps_what_the_last_timed_step_computed(tmp_path):
+  r = _run(['--config', 'c5', '--steps', '3', '--warmup', '3', '--no-cpu-baseline', '--dump-outputs', str(tmp_path)])
+  assert r.returncode == 0, r.stderr[-2000:]
+  d = json.loads(r.stdout)
+  assert d['steps'] == 3
+  names = {'loss', 'masked_weights', 'masks', 'momentum', 'dense_grads', 'other_params'}
+  assert {f for f in os.listdir(tmp_path)} == {n + '.npy' for n in names}
+  assert sum(os.path.getsize(os.path.join(tmp_path, n + '.npy')) for n in names) <= 64 << 20
+  a = {n: np.load(os.path.join(tmp_path, n + '.npy')) for n in names}
+  assert all(v.dtype == np.float32 and np.isfinite(v).all() for v in a.values())
+  assert a['loss'].shape == () and a['loss'] > 0
+  n = a['masked_weights'].size
+  assert n > 0 and all(a[k].size == n for k in ('masks', 'momentum', 'dense_grads'))
+  assert set(np.unique(a['masks'])) == {0.0, 1.0} and abs(a['masks'].mean() - 0.05) < 0.01     # 95 % ERK
+  assert np.count_nonzero(a['dense_grads']) > 0.5 * n                                          # dense, not masked
 
 
 def test_reference_arm_under_torchrun_prints_one_line_from_rank_0():
