@@ -239,6 +239,15 @@ RIGL_API int rigl_masked_conv2d_fprop_bnstats(const rigl_conv_desc* d, const voi
  * <= 128 output channels; otherwise RIGL_ERR_UNSUPPORTED and the caller runs the plain call + a stats pass).
  * on != 0: for every supported shape (tests; same as RIGL_BN_STATS_ALWAYS=1). */
 RIGL_API int rigl_set_bn_stats_always(int on);
+/* Inference: y = [relu](conv(x, mask*W) * scale[c] + shift[c] (+ residual)), bf16 out, fp32 math, one rounding.
+ * scale / shift / residual may be NULL (scale 1, shift 0, no residual); y, scale, shift and residual must be
+ * 16-byte aligned, and residual ([batch,out_h,out_w,cout] bf16) must not overlap y.  RIGL_ERR_UNSUPPORTED where
+ * the shape runs on the halo kernels or where the fused epilogue measured slower than the plain call +
+ * rigl_bn_apply (policy in DESIGN.md 3.8); the caller then runs those two.  RIGL_AFFINE_ALWAYS=1 lifts the
+ * profitability rule (measurement). */
+RIGL_API int rigl_masked_conv2d_fprop_affine(const rigl_conv_desc* d, const void* x, const void* packed,
+                                             const float* scale, const float* shift, const void* residual,
+                                             int relu, void* y_bf16, void* ws, size_t ws_bytes, void* stream);
 /* dx = conv^T(dy, mask*W). */
 RIGL_API int rigl_masked_conv2d_dgrad(const rigl_conv_desc* d, const void* dy, const void* packed,
                                       void* dx, void* ws, size_t ws_bytes, void* stream);
@@ -338,7 +347,7 @@ RIGL_API int rigl_bn_backward2(const void* da, const void* da2, const void* y, c
 /* Max pooling, NHWC bf16, TF 'SAME' padding (out = ceil(in/stride), pad_before = pad_total/2).
  * Replaces tf.layers.max_pooling2d(pool_size=3, strides=2, padding='SAME'),
  * resnet_model.py:636-642.  argmax: one byte per OUTPUT element (window-relative index of the
- * first maximum), consumed by the backward gather.  channels % 8 == 0. */
+ * first maximum), consumed by the backward gather; NULL (inference) skips writing it.  channels % 8 == 0. */
 RIGL_API int rigl_maxpool_same_forward(const void* x, int n, int h, int w, int c, int ksize, int stride,
                                        void* y, uint8_t* argmax, void* stream);
 RIGL_API int rigl_maxpool_same_backward(const void* dy, const uint8_t* argmax, int n, int h, int w, int c,

@@ -74,6 +74,8 @@ SIGNATURES = {
     'rigl_bn_partial_rows': (C.c_int, []),
     'rigl_set_bn_stats_always': (C.c_int, [_i32]),
     'rigl_masked_conv2d_fprop_bnstats': (C.c_int, [C.POINTER(ConvDesc), _vp, _vp, _vp, _vp, C.POINTER(C.c_int), _vp, _sz, _vp]),
+    'rigl_masked_conv2d_fprop_affine': (C.c_int, [C.POINTER(ConvDesc), _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _sz,
+                                                  _vp]),
     'rigl_masked_conv2d_dgrad': (C.c_int, [C.POINTER(ConvDesc), _vp, _vp, _vp, _vp, _sz, _vp]),
     'rigl_conv2d_wgrad_dense': (C.c_int, [C.POINTER(ConvDesc), _vp, _vp, _vp, _f32, _vp, _sz, _vp]),
     'rigl_im2col_nhwc': (C.c_int, [C.POINTER(ConvDesc), _vp, _vp, _i64, _vp]),

@@ -199,6 +199,23 @@ extern "C" int rigl_masked_conv2d_fprop_bnstats(const rigl_conv_desc* d, const v
   return tc_fprop(g, x, packed, y_bf16, nullptr, nullptr, ws, ws_bytes, (cudaStream_t)stream, bn_partial, bn_rows_out);
 }
 
+extern "C" int rigl_masked_conv2d_fprop_affine(const rigl_conv_desc* d, const void* x, const void* packed,
+                                               const float* scale, const float* shift, const void* residual,
+                                               int relu, void* y_bf16, void* ws, size_t ws_bytes, void* stream) {
+  ConvGeom g;
+  int rc = geom_from_desc(d, &g);
+  if (rc != RIGL_OK) return rc;
+  RIGL_REQUIRE(x && packed && y_bf16, "rigl_masked_conv2d_fprop_affine: null tensor");
+  RIGL_REQUIRE(aligned16(y_bf16) && aligned16(scale) && aligned16(shift) && aligned16(residual),
+               "rigl_masked_conv2d_fprop_affine: y, scale, shift and residual must be 16-byte aligned");
+  const AffineEpi epi = {scale, shift, residual, relu ? 1 : 0};
+  const PackedLayout L = packed_layout(g.taps(), g.cin, g.cout);
+  if (!force_simt() && tc_supported(g, 0))
+    return tc_fprop(g, x, packed, y_bf16, nullptr, nullptr, ws, ws_bytes, (cudaStream_t)stream, nullptr, nullptr, &epi);
+  return simt_fprop(g, x, static_cast<const uint8_t*>(packed) + L.off_dgrad, y_bf16, nullptr, nullptr,
+                    (cudaStream_t)stream, &epi);
+}
+
 extern "C" int rigl_masked_conv2d_dgrad(const rigl_conv_desc* d, const void* dy, const void* packed,
                                         void* dx, void* ws, size_t ws_bytes, void* stream) {
   ConvGeom g;

@@ -44,9 +44,17 @@ inline PackedLayout packed_layout(int taps, int cin, int cout) {
 
 int geom_from_desc(const rigl_conv_desc* d, ConvGeom* g);   // validates; sets last error
 
+// Inference epilogue of rigl_masked_conv2d_fprop_affine: y = [relu](acc * scale[c] + shift[c] (+ residual)).
+struct AffineEpi {
+  const float* scale;        // [cout] or null (1)
+  const float* shift;        // [cout] or null (0)
+  const void* residual;      // bf16, the output's shape, or null
+  int relu;
+};
+
 // SIMT path (conv_simt.cu)
 int simt_fprop(const ConvGeom& g, const void* x, const void* w_dgrad, void* y, float* y_f32,
-               const float* bias, cudaStream_t s);
+               const float* bias, cudaStream_t s, const AffineEpi* epi = nullptr);
 int simt_dgrad(const ConvGeom& g, const void* dy, const void* w_fprop, void* dx, cudaStream_t s);
 int simt_wgrad(const ConvGeom& g, const void* x, const void* dy, float* dw, float beta, cudaStream_t s);
 int simt_im2col(const ConvGeom& g, const void* x, void* out, int64_t out_pitch, cudaStream_t s);
@@ -56,7 +64,7 @@ bool tc_supported(const ConvGeom& g, int which /*0 fprop, 1 dgrad, 2 wgrad*/);
 size_t tc_workspace_bytes(const ConvGeom& g);
 int tc_fprop(const ConvGeom& g, const void* x, const void* packed, void* y, float* y_f32,
              const float* bias, void* ws, size_t ws_bytes, cudaStream_t s, float* bn_partial = nullptr,
-             int* bn_rows = nullptr);
+             int* bn_rows = nullptr, const AffineEpi* epi = nullptr);
 int tc_max_ctas();
 void tc_set_bn_stats_always(bool on);
 void tc_set_bn_stats_debug(int v);

@@ -14,9 +14,13 @@ namespace rigl {
 
 // y[p, co] = sum_{tap, ci} x[pix(p, tap), ci] * wd[tap][ci][co]      (wd = w_dgrad layout)
 // grid: (ceil(pixels/4), ceil(cout/64)); block (64, 4)
+// AFF: inference epilogue y = [relu](acc * scale[co] + shift[co] (+ residual[p, co])), one bf16 rounding.
+template <bool AFF>
 __global__ void k_simt_fprop(ConvGeom g, const __nv_bfloat16* __restrict__ x,
                              const __nv_bfloat16* __restrict__ wd, __nv_bfloat16* __restrict__ y,
-                             float* __restrict__ y_f32, const float* __restrict__ bias) {
+                             float* __restrict__ y_f32, const float* __restrict__ bias,
+                             const float* __restrict__ scale, const float* __restrict__ shift,
+                             const __nv_bfloat16* __restrict__ residual, int relu) {
   const int co = blockIdx.y * 64 + threadIdx.x;
   const int64_t p = (int64_t)blockIdx.x * 4 + threadIdx.y;
   if (p >= g.out_pixels() || co >= g.cout) return;
@@ -35,6 +39,11 @@ __global__ void k_simt_fprop(ConvGeom g, const __nv_bfloat16* __restrict__ x,
       for (int ci = 0; ci < g.cin; ++ci)
         acc = fmaf(__bfloat162float(xr[ci]), __bfloat162float(wr[(int64_t)ci * g.cout_pad]), acc);
     }
+  }
+  if constexpr (AFF) {
+    acc = fmaf(acc, scale ? scale[co] : 1.f, shift ? shift[co] : 0.f);
+    if (residual) acc += __bfloat162float(residual[p * g.cout + co]);
+    if (relu) acc = fmaxf(acc, 0.f);
   }
   if (y) y[p * g.cout + co] = __float2bfloat16(acc);
   if (y_f32) y_f32[p * g.cout + co] = acc;
@@ -162,10 +171,15 @@ int simt_im2col(const ConvGeom& g, const void* x, void* out, int64_t out_pitch, 
 }
 
 int simt_fprop(const ConvGeom& g, const void* x, const void* w_dgrad, void* y, float* y_f32,
-               const float* bias, cudaStream_t s) {
+               const float* bias, cudaStream_t s, const AffineEpi* epi) {
   dim3 grid((unsigned)((g.out_pixels() + 3) / 4), (g.cout + 63) / 64), block(64, 4);
-  k_simt_fprop<<<grid, block, 0, s>>>(g, (const __nv_bfloat16*)x, (const __nv_bfloat16*)w_dgrad,
-                                      (__nv_bfloat16*)y, y_f32, bias);
+  if (epi != nullptr)
+    k_simt_fprop<true><<<grid, block, 0, s>>>(g, (const __nv_bfloat16*)x, (const __nv_bfloat16*)w_dgrad,
+                                              (__nv_bfloat16*)y, y_f32, bias, epi->scale, epi->shift,
+                                              (const __nv_bfloat16*)epi->residual, epi->relu);
+  else
+    k_simt_fprop<false><<<grid, block, 0, s>>>(g, (const __nv_bfloat16*)x, (const __nv_bfloat16*)w_dgrad,
+                                               (__nv_bfloat16*)y, y_f32, bias, nullptr, nullptr, nullptr, 0);
   RIGL_LAUNCH_CHECK("k_simt_fprop");
   return RIGL_OK;
 }

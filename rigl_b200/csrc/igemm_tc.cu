@@ -73,6 +73,11 @@ struct IgemmParams {
   float* bn_partial;                // optional [gridDim.x][2][N]: per-CTA column sums / sums of squares of D
   int pair_local;                   // CTA-pair kernel: each CTA's TMA completes on its OWN barrier (see k_igemm_kmajor2)
   int stats_dbg;                    // development: 1 = statistics without the global REDs, 2 = without the smem pass
+  // Inference epilogue (kernel variant AFF = true): y = [relu](acc * scale[c] + shift[c] (+ residual[pixel, c])).
+  const float* ep_scale;            // [N] or null (1)
+  const float* ep_shift;            // [N] or null (0)
+  const __nv_bfloat16* ep_res;      // same shape and pixel offsets as the output, or null
+  int ep_relu;
 };
 
 struct TMaps4 {
@@ -152,12 +157,63 @@ __device__ __forceinline__ void slab_bn_stats(uint32_t slab, int quad, int lane,
   }
 }
 
+// Inference epilogue on one thread's 64 fp32 accumulators of a staged slab (one pixel row, channels co0..co0+63),
+// in place: the folded batch norm, the residual add and the ReLU happen before the single bf16 rounding.  N is a
+// multiple of 8 on this path, so an 8-channel chunk is either wholly inside the output or wholly outside; the scale,
+// shift (16-byte aligned, checked by the caller) and residual row (16-byte loads) are read only for chunks inside it.
+__device__ __forceinline__ void slab_affine(const IgemmParams& p, uint32_t (&r0)[32], uint32_t (&r1)[32], int co0,
+                                            long long o_pix, bool pix_ok) {
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    const int co = co0 + 8 * j;
+    if (co >= p.N) break;
+    float sc[8], sh[8], rs[8];
+    if (p.ep_scale) {
+      const float4 a = __ldg(reinterpret_cast<const float4*>(p.ep_scale + co));
+      const float4 b = __ldg(reinterpret_cast<const float4*>(p.ep_scale + co) + 1);
+      sc[0] = a.x; sc[1] = a.y; sc[2] = a.z; sc[3] = a.w; sc[4] = b.x; sc[5] = b.y; sc[6] = b.z; sc[7] = b.w;
+    } else {
+#pragma unroll
+      for (int e = 0; e < 8; ++e) sc[e] = 1.f;
+    }
+    if (p.ep_shift) {
+      const float4 a = __ldg(reinterpret_cast<const float4*>(p.ep_shift + co));
+      const float4 b = __ldg(reinterpret_cast<const float4*>(p.ep_shift + co) + 1);
+      sh[0] = a.x; sh[1] = a.y; sh[2] = a.z; sh[3] = a.w; sh[4] = b.x; sh[5] = b.y; sh[6] = b.z; sh[7] = b.w;
+    } else {
+#pragma unroll
+      for (int e = 0; e < 8; ++e) sh[e] = 0.f;
+    }
+    uint4 rv = make_uint4(0u, 0u, 0u, 0u);
+    if (p.ep_res && pix_ok) rv = __ldg(reinterpret_cast<const uint4*>(p.ep_res + o_pix + co));
+    const uint32_t rw[4] = {rv.x, rv.y, rv.z, rv.w};
+#pragma unroll
+    for (int e = 0; e < 4; ++e) { rs[2 * e] = __uint_as_float(rw[e] << 16); rs[2 * e + 1] = __uint_as_float(rw[e] & 0xffff0000u); }
+#pragma unroll
+    for (int e = 0; e < 8; ++e) {
+      const int i = 8 * j + e;
+      float z = fmaf(__uint_as_float(i < 32 ? r0[i] : r1[i - 32]), sc[e], sh[e]);
+      if (p.ep_res) z += rs[e];
+      if (p.ep_relu) z = fmaxf(z, 0.f);
+      if (i < 32) r0[i] = __float_as_uint(z); else r1[i - 32] = __float_as_uint(z);
+    }
+  }
+}
+
+// The same transform for one element (the direct-store epilogues: RIGL_TMA_STORE=0).
+__device__ __forceinline__ float elem_affine(const IgemmParams& p, float a, int co, long long o) {
+  float z = fmaf(a, p.ep_scale ? __ldg(p.ep_scale + co) : 1.f, p.ep_shift ? __ldg(p.ep_shift + co) : 0.f);
+  if (p.ep_res) z += __bfloat162float(p.ep_res[o]);
+  return p.ep_relu ? fmaxf(z, 0.f) : z;
+}
+
 // CL = CTAs per cluster (1 or 2).  With CL == 2 the two CTAs work on the two M tiles of a tile
 // PAIR that share the weight tile: each loads HALF of B and multicasts it into both CTAs'
 // shared memory, which cuts the L2->smem bytes per FLOP by a third (these kernels are bound
 // by that traffic, not by the tensor pipe).  A stage is recycled only when BOTH consumers
 // have released it (empty barriers count CL arrivals; tcgen05.commit multicasts them).
-template <int BN, int STAGES, int CL>
+// AFF: the inference epilogue (slab_affine / elem_affine) is compiled in; AFF = false is the training kernel.
+template <int BN, int STAGES, int CL, bool AFF>
 __global__ void __launch_bounds__(kThreads, 1)
 k_igemm_kmajor(const __grid_constant__ TMaps4 amaps, const __grid_constant__ CUtensorMap bmap,
                const __grid_constant__ CUtensorMap omap, const IgemmParams p) {
@@ -319,6 +375,7 @@ k_igemm_kmajor(const __grid_constant__ TMaps4 amaps, const __grid_constant__ CUt
           tmem_ld_32x32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc * BN + c0), r0);
           tmem_ld_32x32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc * BN + c0 + 32), r1);
           tmem_ld_wait();
+          if constexpr (AFF) slab_affine(p, r0, r1, co0, o_pix, pix_ok);
           const uint32_t row_addr = slab + (uint32_t)row * 128u;
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
@@ -363,6 +420,10 @@ k_igemm_kmajor(const __grid_constant__ TMaps4 amaps, const __grid_constant__ CUt
                 for (int q = 0; q < 4; ++q) {
                   float a = __uint_as_float(r[j + 2 * q]), b = __uint_as_float(r[j + 2 * q + 1]);
                   if (p.bias) { a += __ldg(p.bias + co0 + j + 2 * q); b += __ldg(p.bias + co0 + j + 2 * q + 1); }
+                  if constexpr (AFF) {
+                    a = elem_affine(p, a, co0 + j + 2 * q, o_pix + co0 + j + 2 * q);
+                    b = elem_affine(p, b, co0 + j + 2 * q + 1, o_pix + co0 + j + 2 * q + 1);
+                  }
                   __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
                   pk[q] = *reinterpret_cast<uint32_t*>(&h);
                 }
@@ -371,6 +432,7 @@ k_igemm_kmajor(const __grid_constant__ TMaps4 amaps, const __grid_constant__ CUt
                 for (int q = 0; q < 8 && co0 + j + q < p.N; ++q) {
                   float a = __uint_as_float(r[j + q]);
                   if (p.bias) a += __ldg(p.bias + co0 + j + q);
+                  if constexpr (AFF) a = elem_affine(p, a, co0 + j + q, o_pix + co0 + j + q);
                   dst[j + q] = __float2bfloat16(a);
                 }
               }
@@ -448,7 +510,7 @@ struct WgradParams {
 //   * each CTA's epilogue drains its own 128 TMEM lanes and arrives on the leader's
 //     "accumulator free" barrier (count 8).
 // ----------------------------------------------------------------------------
-template <int BN, int STAGES>
+template <int BN, int STAGES, bool AFF>
 __global__ void __launch_bounds__(kThreads, 1)
 k_igemm_kmajor2(const __grid_constant__ TMaps4 amaps, const __grid_constant__ CUtensorMap bmap,
                 const __grid_constant__ CUtensorMap omap, const IgemmParams p) {
@@ -631,6 +693,7 @@ k_igemm_kmajor2(const __grid_constant__ TMaps4 amaps, const __grid_constant__ CU
           tmem_ld_32x32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc * BN + c0), r0);
           tmem_ld_32x32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc * BN + c0 + 32), r1);
           tmem_ld_wait();
+          if constexpr (AFF) slab_affine(p, r0, r1, co0, o_pix, pix_ok);
           const uint32_t row_addr = slab + (uint32_t)row * 128u;
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
@@ -671,6 +734,7 @@ k_igemm_kmajor2(const __grid_constant__ TMaps4 amaps, const __grid_constant__ CU
               if (co0 + j < p.N) {
                 float a = __uint_as_float(r[j]);
                 if (p.bias) a += __ldg(p.bias + co0 + j);
+                if constexpr (AFF) a = elem_affine(p, a, co0 + j, o_pix + co0 + j);
                 if (p.out_bf16) p.out_bf16[o_pix + co0 + j] = __float2bfloat16(a);
                 if (p.out_f32) p.out_f32[o_pix + co0 + j] = a;
               }
@@ -947,6 +1011,7 @@ static bool g_pair_local = false;   // RIGL_PAIR_LOCALBAR=1: per-CTA full barrie
 // spreads over the whole grid.  Kept opt-in as a documented negative result.
 static bool g_wgrad_fixup = false;
 static bool g_bn_stats_always = false;   // RIGL_BN_STATS_ALWAYS=1: epilogue statistics for every supported shape (tests)
+static bool g_affine_always = false;     // RIGL_AFFINE_ALWAYS=1: inference epilogue for every supported shape (measurement)
 static bool g_halo = true;          // RIGL_HALO3X3=0: 3x3/s1 layers with <= 64 channels use the generic kernels
 static int g_halo_t = 0, g_halo_nbuf = 0;   // RIGL_HALO_CFG=T,NBUF: tuning override for the halo kernels
 static bool g_cluster_mc = false;   // RIGL_CLUSTER_MC=1 enables the 2-CTA multicast clusters (measured neutral
@@ -970,6 +1035,7 @@ static void init_driver() {
   if (const char* e = getenv("RIGL_CTA_PAIR")) g_cta_pair = !(e[0] == '0');
   if (const char* e = getenv("RIGL_HALO3X3")) g_halo = !(e[0] == '0');
   if (const char* e = getenv("RIGL_BN_STATS_ALWAYS")) g_bn_stats_always = (e[0] == '1');
+  if (const char* e = getenv("RIGL_AFFINE_ALWAYS")) g_affine_always = (e[0] == '1');
   if (const char* e = getenv("RIGL_WGRAD_FIXUP")) g_wgrad_fixup = (e[0] == '1');
   if (const char* e = getenv("RIGL_PAIR_LOCALBAR")) g_pair_local = (e[0] == '1');
   if (const char* e = getenv("RIGL_HALO_CFG")) sscanf(e, "%d,%d", &g_halo_t, &g_halo_nbuf);
@@ -1116,13 +1182,13 @@ static int kmajor_grid(const IgemmParams& p) {         // CTAs the K-major launc
   return clusters * cl;
 }
 
-template <int BN, int STAGES, int CL>
+template <int BN, int STAGES, int CL, bool AFF>
 static int launch_kmajor(const TMaps4& amaps, const CUtensorMap& bmap, const CUtensorMap& omap, const IgemmParams& p,
                          cudaStream_t s) {
   constexpr size_t smem = (size_t)STAGES * (kBM * kBK * 2 + BN * kBK * 2) + 2 * (kBM * 64 * 2) + 1024 + 256;
   static bool configured = false;
   if (!configured) {
-    RIGL_CUDA(cudaFuncSetAttribute(k_igemm_kmajor<BN, STAGES, CL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    RIGL_CUDA(cudaFuncSetAttribute(k_igemm_kmajor<BN, STAGES, CL, AFF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured = true;
   }
   const int m_tiles = p.tiles_w * p.tiles_h * p.tiles_n;
@@ -1140,21 +1206,21 @@ static int launch_kmajor(const TMaps4& amaps, const CUtensorMap& bmap, const CUt
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   if (CL == 1) {
-    k_igemm_kmajor<BN, STAGES, CL><<<cfg.gridDim, cfg.blockDim, smem, s>>>(amaps, bmap, omap, p);
+    k_igemm_kmajor<BN, STAGES, CL, AFF><<<cfg.gridDim, cfg.blockDim, smem, s>>>(amaps, bmap, omap, p);
   } else {
-    RIGL_CUDA(cudaLaunchKernelEx(&cfg, k_igemm_kmajor<BN, STAGES, CL>, amaps, bmap, omap, p));
+    RIGL_CUDA(cudaLaunchKernelEx(&cfg, k_igemm_kmajor<BN, STAGES, CL, AFF>, amaps, bmap, omap, p));
   }
   RIGL_LAUNCH_CHECK("k_igemm_kmajor");
   return RIGL_OK;
 }
 
-template <int BN, int STAGES>
+template <int BN, int STAGES, bool AFF>
 static int launch_kmajor2(const TMaps4& amaps, const CUtensorMap& bmap, const CUtensorMap& omap, const IgemmParams& p,
                           cudaStream_t s) {
   constexpr size_t smem = (size_t)STAGES * (kBM * kBK * 2 + (BN / 2) * kBK * 2) + 2 * (kBM * 64 * 2) + 1024 + 512;
   static bool configured = false;
   if (!configured) {
-    RIGL_CUDA(cudaFuncSetAttribute(k_igemm_kmajor2<BN, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    RIGL_CUDA(cudaFuncSetAttribute(k_igemm_kmajor2<BN, STAGES, AFF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured = true;
   }
   const int m_tiles = p.tiles_w * p.tiles_h * p.tiles_n;
@@ -1171,24 +1237,32 @@ static int launch_kmajor2(const TMaps4& amaps, const CUtensorMap& bmap, const CU
   attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  RIGL_CUDA(cudaLaunchKernelEx(&cfg, k_igemm_kmajor2<BN, STAGES>, amaps, bmap, omap, p));
+  RIGL_CUDA(cudaLaunchKernelEx(&cfg, k_igemm_kmajor2<BN, STAGES, AFF>, amaps, bmap, omap, p));
   RIGL_LAUNCH_CHECK("k_igemm_kmajor2");
   return RIGL_OK;
 }
 
-static int dispatch_kmajor(int n_out, const TMaps4& amaps, const CUtensorMap& bmap, const CUtensorMap& omap,
-                           IgemmParams& p, int bn_tile, cudaStream_t s) {
+template <bool AFF>
+static int dispatch_kmajor_t(int n_out, const TMaps4& amaps, const CUtensorMap& bmap, const CUtensorMap& omap,
+                             IgemmParams& p, int bn_tile, cudaStream_t s) {
   p.n_tiles = (n_out + bn_tile - 1) / bn_tile;
   if (kmajor_use_pair(p)) {               // CTA-pair MMA (M = 256); bmap was built with bn_tile/2 rows
     p.pair_local = g_pair_local ? 1 : 0;
-    if (bn_tile == 64) return launch_kmajor2<64, 9>(amaps, bmap, omap, p, s);
-    if (bn_tile == 128) return launch_kmajor2<128, 8>(amaps, bmap, omap, p, s);
-    return launch_kmajor2<256, 6>(amaps, bmap, omap, p, s);
+    if (bn_tile == 64) return launch_kmajor2<64, 9, AFF>(amaps, bmap, omap, p, s);
+    if (bn_tile == 128) return launch_kmajor2<128, 8, AFF>(amaps, bmap, omap, p, s);
+    return launch_kmajor2<256, 6, AFF>(amaps, bmap, omap, p, s);
   }
   const bool mc = kmajor_use_mc(p);                        // multicast needs a partner M tile
-  if (bn_tile == 64) return mc ? launch_kmajor<64, 8, 2>(amaps, bmap, omap, p, s) : launch_kmajor<64, 8, 1>(amaps, bmap, omap, p, s);
-  if (bn_tile == 128) return mc ? launch_kmajor<128, 6, 2>(amaps, bmap, omap, p, s) : launch_kmajor<128, 6, 1>(amaps, bmap, omap, p, s);
-  return mc ? launch_kmajor<256, 4, 2>(amaps, bmap, omap, p, s) : launch_kmajor<256, 4, 1>(amaps, bmap, omap, p, s);
+  if (bn_tile == 64) return mc ? launch_kmajor<64, 8, 2, AFF>(amaps, bmap, omap, p, s) : launch_kmajor<64, 8, 1, AFF>(amaps, bmap, omap, p, s);
+  if (bn_tile == 128) return mc ? launch_kmajor<128, 6, 2, AFF>(amaps, bmap, omap, p, s) : launch_kmajor<128, 6, 1, AFF>(amaps, bmap, omap, p, s);
+  return mc ? launch_kmajor<256, 4, 2, AFF>(amaps, bmap, omap, p, s) : launch_kmajor<256, 4, 1, AFF>(amaps, bmap, omap, p, s);
+}
+
+// affine: the inference-epilogue kernel variant (p.ep_*), a separate instantiation of every K-major kernel.
+static int dispatch_kmajor(int n_out, const TMaps4& amaps, const CUtensorMap& bmap, const CUtensorMap& omap,
+                           IgemmParams& p, int bn_tile, cudaStream_t s, bool affine = false) {
+  return affine ? dispatch_kmajor_t<true>(n_out, amaps, bmap, omap, p, bn_tile, s)
+                : dispatch_kmajor_t<false>(n_out, amaps, bmap, omap, p, bn_tile, s);
 }
 
 static int pick_bn(int n_out, long long m_tiles) {
@@ -1202,8 +1276,18 @@ void tc_set_bn_stats_always(bool on) { g_bn_stats_always = on; }
 static int g_stats_dbg = 0;
 void tc_set_bn_stats_debug(int v) { g_stats_dbg = v; }
 
+// Measured on B200 (ResNet-50 and MobileNet-v1 at b256, profiles/r03_inference_shapes.md), fused call against the plain
+// call + rigl_bn_apply: with a residual the per-thread 16-byte loads of the shortcut rows make the epilogue the
+// bottleneck, 1.52-1.79x on every ResNet-50 shape that has one; without a residual the fused call takes 0.73-0.92x,
+// except the short-K, wide output on a small pixel grid (7x7 512->1024, K = 512: 1.065x, runs within 1 %).
+static bool affine_profitable(const ConvGeom& g, const AffineEpi& e) {
+  if (e.residual != nullptr) return false;
+  const int K = g.taps() * g.cin;
+  return !(K <= 512 && g.cout >= 2 * K && g.out_pixels() <= 12544);
+}
+
 int tc_fprop(const ConvGeom& g, const void* x, const void* packed, void* y, float* y_f32, const float* bias,
-             void* ws, size_t ws_bytes, cudaStream_t s, float* bn_partial, int* bn_rows) {
+             void* ws, size_t ws_bytes, cudaStream_t s, float* bn_partial, int* bn_rows, const AffineEpi* epi) {
   (void)ws; (void)ws_bytes;
   int rc = ensure_driver();
   if (rc != RIGL_OK) return rc;
@@ -1214,6 +1298,10 @@ int tc_fprop(const ConvGeom& g, const void* x, const void* packed, void* y, floa
     if (y != nullptr && y_f32 == nullptr && bias == nullptr && halo_fprop_ok(g, &hp)) {
       if (bn_partial != nullptr) {        // the halo kernels have no statistics epilogue: the caller runs the plain
         set_error("fused BN statistics: layer runs on the halo kernels");   // call + the stats pass instead
+        return RIGL_ERR_UNSUPPORTED;
+      }
+      if (epi != nullptr) {               // nor an inference epilogue: plain call + rigl_bn_apply
+        set_error("fused inference epilogue: layer runs on the halo kernels");
         return RIGL_ERR_UNSUPPORTED;
       }
       return halo_launch_kmajor(hp, x, g.cin, g.x_pitch, pk + L.off_fprop, L.cin_pad, g.cout, y, g.cout, false, s);
@@ -1230,6 +1318,11 @@ int tc_fprop(const ConvGeom& g, const void* x, const void* packed, void* y, floa
       return RIGL_ERR_UNSUPPORTED;
     }
   }
+  if (epi != nullptr && !g_affine_always && !affine_profitable(g, *epi)) {
+    set_error("fused inference epilogue: not profitable for this shape (K = %d, cout = %d, residual %d)",
+              g.taps() * g.cin, g.cout, epi->residual != nullptr);
+    return RIGL_ERR_UNSUPPORTED;
+  }
   IgemmParams p = {};
   choose_box(g.out_w, g.out_h, g.batch, 128, &p.bw, &p.bh, &p.bn);
   p.GW = g.out_w; p.GH = g.out_h; p.NB = g.batch;
@@ -1237,6 +1330,10 @@ int tc_fprop(const ConvGeom& g, const void* x, const void* packed, void* y, floa
   p.kblks = (g.cin + kBK - 1) / kBK;
   p.N = g.cout;
   p.out_bf16 = static_cast<__nv_bfloat16*>(y); p.out_f32 = y_f32; p.bias = bias;
+  if (epi != nullptr) {
+    p.ep_scale = epi->scale; p.ep_shift = epi->shift; p.ep_relu = epi->relu;
+    p.ep_res = static_cast<const __nv_bfloat16*>(epi->residual);
+  }
   p.o_off = 0; p.o_sw = g.cout; p.o_sh = (long long)g.out_w * g.cout; p.o_sn = (long long)g.out_h * g.out_w * g.cout;
   p.nnz = reinterpret_cast<const uint32_t*>(pk + L.off_nnz);
   p.nnz_tap_stride = L.n_tiles * L.k_tiles; p.nnz_n_stride = L.k_tiles; p.nnz_k_stride = 1;
@@ -1282,7 +1379,7 @@ int tc_fprop(const ConvGeom& g, const void* x, const void* packed, void* y, floa
     p.n_tiles = (g.cout + bn_tile - 1) / bn_tile;
     if (bn_rows) *bn_rows = kmajor_grid(p);
   }
-  return dispatch_kmajor(g.cout, amaps, bmap, omap, p, bn_tile, s);
+  return dispatch_kmajor(g.cout, amaps, bmap, omap, p, bn_tile, s, epi != nullptr);
 }
 
 int tc_dgrad(const ConvGeom& g, const void* dy, const void* packed, void* dx, void* ws, size_t ws_bytes,

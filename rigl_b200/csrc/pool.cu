@@ -15,6 +15,8 @@ struct PoolGeom {
   int n, h, w, c, oh, ow, k, s, pad;
 };
 
+// kArg = false: inference (no backward pass follows), the argmax bytes are not written.
+template <bool kArg>
 __global__ void __launch_bounds__(256)
 k_maxpool_fwd(PoolGeom g, const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __restrict__ y,
               uint8_t* __restrict__ idx) {
@@ -50,10 +52,12 @@ k_maxpool_fwd(PoolGeom g, const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __
 #pragma unroll
     for (int e = 0; e < 4; ++e) oh2[e] = __floats2bfloat162_rn(best[2 * e], best[2 * e + 1]);
     *reinterpret_cast<uint4*>(y + p * g.c + 8 * v) = o;
-    uint2 a;
-    a.x = arg[0] | (arg[1] << 8) | (arg[2] << 16) | ((uint32_t)arg[3] << 24);
-    a.y = arg[4] | (arg[5] << 8) | (arg[6] << 16) | ((uint32_t)arg[7] << 24);
-    *reinterpret_cast<uint2*>(idx + p * g.c + 8 * v) = a;
+    if constexpr (kArg) {
+      uint2 a;
+      a.x = arg[0] | (arg[1] << 8) | (arg[2] << 16) | ((uint32_t)arg[3] << 24);
+      a.y = arg[4] | (arg[5] << 8) | (arg[6] << 16) | ((uint32_t)arg[7] << 24);
+      *reinterpret_cast<uint2*>(idx + p * g.c + 8 * v) = a;
+    }
   }
 }
 
@@ -169,10 +173,13 @@ extern "C" int rigl_maxpool_same_forward(const void* x, int n, int h, int w, int
   PoolGeom g;
   int rc = pool_geom(n, h, w, c, ksize, stride, &g);
   if (rc != RIGL_OK) return rc;
-  RIGL_REQUIRE(x && y && argmax, "rigl_maxpool_same_forward: null tensor");
+  RIGL_REQUIRE(x && y, "rigl_maxpool_same_forward: null tensor");
   RIGL_REQUIRE(g.oh <= 65535 && n <= 65535, "rigl_maxpool_same_forward: extent too large");
   const dim3 block(8, 32), grid((unsigned)((g.ow + 31) / 32), (unsigned)g.oh, (unsigned)n);
-  k_maxpool_fwd<<<grid, block, 0, (cudaStream_t)stream>>>(g, (const __nv_bfloat16*)x, (__nv_bfloat16*)y, argmax);
+  if (argmax)
+    k_maxpool_fwd<true><<<grid, block, 0, (cudaStream_t)stream>>>(g, (const __nv_bfloat16*)x, (__nv_bfloat16*)y, argmax);
+  else
+    k_maxpool_fwd<false><<<grid, block, 0, (cudaStream_t)stream>>>(g, (const __nv_bfloat16*)x, (__nv_bfloat16*)y, nullptr);
   RIGL_LAUNCH_CHECK("k_maxpool_fwd");
   return RIGL_OK;
 }
