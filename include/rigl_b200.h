@@ -223,7 +223,9 @@ typedef struct {
 
 RIGL_API size_t rigl_conv_workspace_bytes(const rigl_conv_desc* d);
 /* y = conv(x, mask*W) (+ bias[cout]).  `packed` from rigl_pack_masked_weights.
- * y_bf16 and/or y_f32 receive the result (either may be NULL, not both). */
+ * y_bf16 and/or y_f32 receive the result (either may be NULL, not both).  On the tensor-core path
+ * (cout and x_pitch multiples of 8) both must be 16-byte aligned: the epilogue writes 16-byte
+ * vectors (RIGL_ERR_INVALID_ARG otherwise; the same holds for dx of rigl_masked_conv2d_dgrad). */
 RIGL_API int rigl_masked_conv2d_fprop(const rigl_conv_desc* d, const void* x, const void* packed,
                                       void* y_bf16, float* y_f32, const float* bias, void* ws,
                                       size_t ws_bytes, void* stream);
@@ -261,7 +263,7 @@ RIGL_API int rigl_conv2d_wgrad_dense(const rigl_conv_desc* d, const void* x, con
  * runs as a masked dense layer over [pixels, k*k*cin] with the SAME HWIO weights and mask. */
 RIGL_API int rigl_im2col_nhwc(const rigl_conv_desc* d, const void* x, void* out, int64_t out_pitch,
                               void* stream);
-/* EXPERIMENTAL (opt-in in the host mirror: layers.STEM_S2D_PATH; not yet validated on hardware).
+/* Space-to-depth stem (the default for this shape in the host mirror: layers.STEM_S2D_PATH).
  * The 7x7 / stride-2 / 3-channel stem (conv2d_fixed_padding, resnet_model.py:619-629) without a
  * patch matrix: rigl_stem_s2d_fold_input folds the zero-padded input 2x2 -> 16 channels
  * ([N,(H+6)/2,(W+6)/2,16] bf16, rigl_stem_s2d_folded_bytes), the conv becomes a 4x4 stride-1 conv
@@ -280,24 +282,6 @@ RIGL_API int rigl_stem_s2d_fprop(const rigl_conv_desc* d, const void* xs, const 
                                  void* stream);
 RIGL_API int rigl_stem_s2d_wgrad(const rigl_conv_desc* d, const void* xs, const void* dy, float* dw,
                                  float beta, void* ws, size_t ws_bytes, void* stream);
-
-/* Small-Cin convs (cin <= 8, ksize <= 8: the 7x7x3 stem, resnet_model.py:620-633) WITHOUT a
- * patch matrix: the input is copied once into a zero-bordered 8-channel buffer `xp`
- * (rigl_smallc_padded_bytes); window tensor maps with a W stride of `stride` pixels then feed
- * the same tcgen05 kernels with ksize "taps" of K = 64 = 8 pixels x 8 channels.  `packed` here
- * is the stem-specific operand written by rigl_smallc_pack_weights from the SAME HWIO weights
- * and mask.  dw is the dense HWIO gradient as in rigl_conv2d_wgrad_dense. */
-RIGL_API int rigl_smallc_supported(const rigl_conv_desc* d);
-RIGL_API size_t rigl_smallc_padded_bytes(const rigl_conv_desc* d);
-RIGL_API size_t rigl_smallc_packed_bytes(const rigl_conv_desc* d);
-RIGL_API size_t rigl_smallc_workspace_bytes(const rigl_conv_desc* d);
-RIGL_API int rigl_smallc_pad_input(const rigl_conv_desc* d, const void* x, void* xp, void* stream);
-RIGL_API int rigl_smallc_pack_weights(const rigl_conv_desc* d, const float* w_hwio,
-                                      const uint32_t* mask_bits, void* packed, void* stream);
-RIGL_API int rigl_smallc_fprop(const rigl_conv_desc* d, const void* xp, const void* packed, void* y,
-                               void* stream);
-RIGL_API int rigl_smallc_wgrad(const rigl_conv_desc* d, const void* xp, const void* dy, float* dw,
-                               float beta, void* ws, size_t ws_bytes, void* stream);
 
 /* ------------------------------------------------------------------------
  * Fused batch-norm (+ReLU, +residual) over NHWC bf16 activations viewed as [rows, channels]

@@ -87,14 +87,6 @@ SIGNATURES = {
     'rigl_stem_s2d_pack_weights': (C.c_int, [C.POINTER(ConvDesc), _vp, _vp, _vp, _vp]),
     'rigl_stem_s2d_fprop': (C.c_int, [C.POINTER(ConvDesc), _vp, _vp, _vp, _vp]),
     'rigl_stem_s2d_wgrad': (C.c_int, [C.POINTER(ConvDesc), _vp, _vp, _vp, _f32, _vp, _sz, _vp]),
-    'rigl_smallc_supported': (C.c_int, [C.POINTER(ConvDesc)]),
-    'rigl_smallc_padded_bytes': (_sz, [C.POINTER(ConvDesc)]),
-    'rigl_smallc_packed_bytes': (_sz, [C.POINTER(ConvDesc)]),
-    'rigl_smallc_workspace_bytes': (_sz, [C.POINTER(ConvDesc)]),
-    'rigl_smallc_pad_input': (C.c_int, [C.POINTER(ConvDesc), _vp, _vp, _vp]),
-    'rigl_smallc_pack_weights': (C.c_int, [C.POINTER(ConvDesc), _vp, _vp, _vp, _vp]),
-    'rigl_smallc_fprop': (C.c_int, [C.POINTER(ConvDesc), _vp, _vp, _vp, _vp]),
-    'rigl_smallc_wgrad': (C.c_int, [C.POINTER(ConvDesc), _vp, _vp, _vp, _f32, _vp, _sz, _vp]),
     'rigl_bn_workspace_bytes': (_sz, [_i64, _i32]),
     'rigl_bn_forward_train': (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i32, _f32, _f32, _i32, _vp, _vp, _vp, _vp,
                                         _vp, _vp, _vp, _vp, _sz, _vp, _vp]),

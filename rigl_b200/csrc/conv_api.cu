@@ -52,8 +52,7 @@ extern "C" int rigl_im2col_nhwc(const rigl_conv_desc* d, const void* x, void* ou
   return simt_im2col(g, x, out, out_pitch, (cudaStream_t)stream);
 }
 
-// ---- small-Cin (stem) convs: zero-bordered 8-channel input + window tensor maps ----
-// ---- space-to-depth stem (experimental, see stem_s2d.cuh) ----
+// ---- space-to-depth stem (7x7 / stride 2 / <= 3 channels, see stem_s2d.cuh) ----
 extern "C" int rigl_stem_s2d_supported(const rigl_conv_desc* d) {
   ConvGeom g;
   if (geom_from_desc(d, &g) != RIGL_OK) return 0;
@@ -103,55 +102,6 @@ extern "C" int rigl_stem_s2d_wgrad(const rigl_conv_desc* d, const void* xs, cons
   return s2d_wgrad(g, xs, dy, dw, beta, ws, ws_bytes, (cudaStream_t)stream);
 }
 
-extern "C" int rigl_smallc_supported(const rigl_conv_desc* d) {
-  ConvGeom g;
-  if (geom_from_desc(d, &g) != RIGL_OK) return 0;
-  return smallc_supported(g) && !force_simt() ? 1 : 0;
-}
-extern "C" size_t rigl_smallc_padded_bytes(const rigl_conv_desc* d) {
-  ConvGeom g;
-  return geom_from_desc(d, &g) == RIGL_OK ? smallc_padded_bytes(g) : 0;
-}
-extern "C" size_t rigl_smallc_packed_bytes(const rigl_conv_desc* d) {
-  ConvGeom g;
-  return geom_from_desc(d, &g) == RIGL_OK ? smallc_packed_bytes(g) : 0;
-}
-extern "C" size_t rigl_smallc_workspace_bytes(const rigl_conv_desc* d) {
-  ConvGeom g;
-  return geom_from_desc(d, &g) == RIGL_OK ? smallc_wgrad_ws_bytes(g) : 0;
-}
-extern "C" int rigl_smallc_pad_input(const rigl_conv_desc* d, const void* x, void* xp, void* stream) {
-  ConvGeom g;
-  int rc = geom_from_desc(d, &g);
-  if (rc != RIGL_OK) return rc;
-  RIGL_REQUIRE(x && xp && smallc_supported(g) && aligned16(xp), "rigl_smallc_pad_input: bad arguments");
-  return smallc_pad_input(g, x, xp, (cudaStream_t)stream);
-}
-extern "C" int rigl_smallc_pack_weights(const rigl_conv_desc* d, const float* w_hwio, const uint32_t* mask_bits,
-                                        void* packed, void* stream) {
-  ConvGeom g;
-  int rc = geom_from_desc(d, &g);
-  if (rc != RIGL_OK) return rc;
-  RIGL_REQUIRE(w_hwio && mask_bits && packed && smallc_supported(g), "rigl_smallc_pack_weights: bad arguments");
-  return smallc_pack(g, w_hwio, mask_bits, packed, (cudaStream_t)stream);
-}
-extern "C" int rigl_smallc_fprop(const rigl_conv_desc* d, const void* xp, const void* packed, void* y,
-                                 void* stream) {
-  ConvGeom g;
-  int rc = geom_from_desc(d, &g);
-  if (rc != RIGL_OK) return rc;
-  RIGL_REQUIRE(xp && packed && y && smallc_supported(g), "rigl_smallc_fprop: bad arguments");
-  return smallc_fprop(g, xp, packed, y, (cudaStream_t)stream);
-}
-extern "C" int rigl_smallc_wgrad(const rigl_conv_desc* d, const void* xp, const void* dy, float* dw, float beta,
-                                 void* ws, size_t ws_bytes, void* stream) {
-  ConvGeom g;
-  int rc = geom_from_desc(d, &g);
-  if (rc != RIGL_OK) return rc;
-  RIGL_REQUIRE(xp && dy && dw && smallc_supported(g), "rigl_smallc_wgrad: bad arguments");
-  return smallc_wgrad(g, xp, dy, dw, beta, ws, ws_bytes, (cudaStream_t)stream);
-}
-
 extern "C" int rigl_set_force_simt(int on) {
   g_force_simt = on ? 1 : 0;
   return RIGL_OK;
@@ -171,8 +121,10 @@ extern "C" int rigl_masked_conv2d_fprop(const rigl_conv_desc* d, const void* x, 
   if (rc != RIGL_OK) return rc;
   RIGL_REQUIRE(x && packed && (y_bf16 || y_f32), "rigl_masked_conv2d_fprop: null tensor");
   const PackedLayout L = packed_layout(g.taps(), g.cin, g.cout);
-  if (!force_simt() && tc_supported(g, 0))
+  if (!force_simt() && tc_supported(g, 0)) {
+    RIGL_REQUIRE(aligned16(y_bf16) && aligned16(y_f32), "rigl_masked_conv2d_fprop: y_bf16 and y_f32 must be 16-byte aligned");
     return tc_fprop(g, x, packed, y_bf16, y_f32, bias, ws, ws_bytes, (cudaStream_t)stream);
+  }
   return simt_fprop(g, x, static_cast<const uint8_t*>(packed) + L.off_dgrad, y_bf16, y_f32, bias,
                     (cudaStream_t)stream);
 }
@@ -181,7 +133,6 @@ extern "C" int rigl_bn_partial_rows(void) { return tc_max_ctas(); }
 
 extern "C" int rigl_set_bn_stats_always(int on) {
   tc_set_bn_stats_always(on != 0);
-  tc_set_bn_stats_debug(on >> 4);       // (development: bits 4.. select partial variants of the statistics code)
   return RIGL_OK;
 }
 
@@ -223,8 +174,10 @@ extern "C" int rigl_masked_conv2d_dgrad(const rigl_conv_desc* d, const void* dy,
   if (rc != RIGL_OK) return rc;
   RIGL_REQUIRE(dy && packed && dx, "rigl_masked_conv2d_dgrad: null tensor");
   const PackedLayout L = packed_layout(g.taps(), g.cin, g.cout);
-  if (!force_simt() && tc_supported(g, 1))
+  if (!force_simt() && tc_supported(g, 1)) {
+    RIGL_REQUIRE(aligned16(dx), "rigl_masked_conv2d_dgrad: dx must be 16-byte aligned");
     return tc_dgrad(g, dy, packed, dx, ws, ws_bytes, (cudaStream_t)stream);
+  }
   return simt_dgrad(g, dy, static_cast<const uint8_t*>(packed) + L.off_fprop, dx, (cudaStream_t)stream);
 }
 

@@ -67,14 +67,12 @@ int tc_fprop(const ConvGeom& g, const void* x, const void* packed, void* y, floa
              int* bn_rows = nullptr, const AffineEpi* epi = nullptr);
 int tc_max_ctas();
 void tc_set_bn_stats_always(bool on);
-void tc_set_bn_stats_debug(int v);
 int tc_dgrad(const ConvGeom& g, const void* dy, const void* packed, void* dx, void* ws,
              size_t ws_bytes, cudaStream_t s);
 int tc_wgrad(const ConvGeom& g, const void* x, const void* dy, float* dw, float beta, void* ws,
              size_t ws_bytes, cudaStream_t s);
 
-// small-Cin (stem) path (igemm_tc.cu)
-// Space-to-depth stem (stem_s2d.cuh) -- experimental, opt-in
+// Space-to-depth stem (stem_s2d.cuh, included by igemm_tc.cu)
 bool s2d_supported(const ConvGeom& g);
 size_t s2d_folded_bytes(const ConvGeom& g);
 size_t s2d_packed_bytes(const ConvGeom& g);
@@ -84,14 +82,5 @@ int s2d_pack(const ConvGeom& g, const float* w, const uint32_t* bits, void* pack
 int s2d_fprop(const ConvGeom& g, const void* xs, const void* packed, void* y, cudaStream_t s);
 int s2d_wgrad(const ConvGeom& g, const void* xs, const void* dy, float* dw, float beta, void* ws, size_t ws_bytes,
               cudaStream_t s);
-bool smallc_supported(const ConvGeom& g);
-size_t smallc_padded_bytes(const ConvGeom& g);
-size_t smallc_packed_bytes(const ConvGeom& g);
-size_t smallc_wgrad_ws_bytes(const ConvGeom& g);
-int smallc_pad_input(const ConvGeom& g, const void* x, void* xp, cudaStream_t s);
-int smallc_pack(const ConvGeom& g, const float* w, const uint32_t* bits, void* packed, cudaStream_t s);
-int smallc_fprop(const ConvGeom& g, const void* xp, const void* packed, void* y, cudaStream_t s);
-int smallc_wgrad(const ConvGeom& g, const void* xp, const void* dy, float* dw, float beta, void* ws,
-                 size_t ws_bytes, cudaStream_t s);
 
 }  // namespace rigl

@@ -141,23 +141,7 @@ k_halo3x3_kmajor(const __grid_constant__ CUtensorMap amap, const __grid_constant
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(tempty_bar(acc));       // accumulator drained into registers
-        const uint32_t row_addr = slab + (uint32_t)row * 128u;
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          uint32_t pk[4];
-#pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            const int e = 8 * j + 2 * q;
-            const float a = __uint_as_float(e < 32 ? r0[e] : r1[e - 32]);
-            const float b = __uint_as_float(e + 1 < 32 ? r0[e + 1] : r1[e + 1 - 32]);
-            __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-            pk[q] = *reinterpret_cast<uint32_t*>(&h);
-          }
-          const uint32_t dst = row_addr + (uint32_t)((j ^ (row & 7)) << 4);
-          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst), "r"(pk[0]), "r"(pk[1]), "r"(pk[2]),
-                       "r"(pk[3])
-                       : "memory");
-        }
+        stage_row_bf16(slab, row, r0, r1, false);
         fence_proxy_async_smem();
         named_bar_sync(1, 128);
         if (issuer) {                                      // columns >= W and rows >= H are clipped by TMA
@@ -338,13 +322,6 @@ static bool halo_geom(const ConvGeom& g, int kred, HaloParams* p, size_t smem_fi
       if (r >= g.in_h) break;
     }
   if (best_t == 0) return false;
-  if (g_halo_t > 0 && g_halo_nbuf >= 2 && g_halo_nbuf <= 4) {        // experiment override (RIGL_HALO_CFG=T,NBUF)
-    const int r = rt * g_halo_t;
-    const size_t a_buf = ((size_t)((r + 2) * wp + 8) * 128 + 1023) / 1024 * 1024;
-    if (smem_fixed + g_halo_nbuf * (a_buf + (dy_tile ? (size_t)r * wp * 128 : 0)) + 2048 <= 227 * 1024) {
-      best_t = g_halo_t; best_nbuf = g_halo_nbuf;
-    }
-  }
   p->W = g.in_w; p->H = g.in_h; p->NB = g.batch; p->Wp = wp;
   p->T = best_t; p->R = rt * best_t; p->nbuf = best_nbuf;
   p->strips_per_image = (g.in_h + p->R - 1) / p->R;

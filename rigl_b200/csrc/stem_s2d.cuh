@@ -191,23 +191,7 @@ k_stem_s2d_fprop(const __grid_constant__ CUtensorMap amap, const __grid_constant
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(tempty_bar(acc));
-        const uint32_t row_addr = slab + (uint32_t)row * 128u;
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          uint32_t pk[4];
-#pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            const int e = 8 * j + 2 * q;
-            const float a = __uint_as_float(e < 32 ? r0[e] : r1[e - 32]);
-            const float b = __uint_as_float(e + 1 < 32 ? r0[e + 1] : r1[e + 1 - 32]);
-            __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-            pk[q] = *reinterpret_cast<uint32_t*>(&h);
-          }
-          const uint32_t dst = row_addr + (uint32_t)((j ^ (row & 7)) << 4);
-          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst), "r"(pk[0]), "r"(pk[1]), "r"(pk[2]),
-                       "r"(pk[3])
-                       : "memory");
-        }
+        stage_row_bf16(slab, row, r0, r1, false);
         fence_proxy_async_smem();
         named_bar_sync(1, 128);
         if (issuer) {                                        // columns >= W and rows >= H are clipped by TMA

@@ -85,22 +85,6 @@ __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* m, 
       : "memory");
 }
 
-// Multicast variants: the box is written at the same CTA-relative smem offset of every CTA in
-// `mask`, and complete_tx is signalled on the mbarrier at the same offset in each of them.
-__device__ __forceinline__ void tma_load_3d_mc(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1,
-                                               int c2, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4, %5}], [%2], %6;"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "h"(mask)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_4d_mc(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1,
-                                               int c2, int c3, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4, %5, %6}], [%2], %7;"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "h"(mask)
-      : "memory");
-}
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -134,32 +118,6 @@ __device__ __forceinline__ void tma_load_3d_2cta(uint32_t dst, const CUtensorMap
 // Arrive (no tx) on the LEADER CTA's barrier from either CTA of the pair.
 __device__ __forceinline__ void mbar_arrive_leader(uint32_t bar) {
   asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(bar & kPeerBitMask) : "memory");
-}
-// Cluster-scope release / acquire pair for a hand-off that crosses the CTA pair
-// (peer: data landed in MY shared memory -> leader: may now issue the pair MMA that reads it).
-__device__ __forceinline__ void mbar_arrive_leader_release(uint32_t bar) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar & kPeerBitMask) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
-  uint32_t done;
-  uint32_t spins = 0;
-  long long t0 = 0;
-  do {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n"
-        "selp.u32 %0, 1, 0, p;\n"
-        "}\n"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    if (!done && (++spins & 0xFFFu) == 0) {
-      const long long now = clock64();
-      if (t0 == 0) t0 = now;
-      else if (now - t0 > 8000000000ll) __trap();
-    }
-  } while (!done);
 }
 __device__ __forceinline__ void tmem_alloc_2cta(uint32_t smem_dst, uint32_t ncols) {   // one warp in EACH CTA
   asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(ncols)
@@ -235,12 +193,6 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t desc_a, uint
 // mbarrier arrives when all previously issued MMAs of this thread have completed.
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar)
-               : "memory");
-}
-// Same, arriving on the barrier at this offset in every CTA of `mask` (cluster multicast).
-__device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-               "h"(mask)
                : "memory");
 }
 // 32 lanes x 32 consecutive fp32 columns -> 32 registers per thread (lane = TMEM lane).

@@ -40,7 +40,6 @@ def _bn_partial_rows():
   return _BN_ROWS[0]
 
 
-STEM_WINDOW_PATH = False     # route small-Cin convs through the window-tensor-map kernels
 # space-to-depth halo kernels for the 7x7/2 3-channel stem (csrc/stem_s2d.cuh, DESIGN.md 3.7): validated on
 # B200 at the start of round 2 (tools/umma_sw32_probe.cu + tests/test_conv_gpu.py::test_conv_stem_s2d_path);
 # RIGL_STEM_S2D=0 falls back to the patch-matrix (im2col) stem
@@ -177,7 +176,7 @@ class PackPlan(object):
       self._plan, self._key = plan, key
     _cabi.check(_cabi.lib().rigl_pack_plan_run(self._plan, _cabi.stream_ptr()), 'rigl_pack_plan_run')
     for l in layers:          # the small special-format stem operands are not part of the batch
-      if getattr(l, 's2d_mode', False) or getattr(l, 'smallc_mode', False):
+      if getattr(l, 's2d_mode', False):
         l.pack_special()
 
 
@@ -362,19 +361,11 @@ class SparseConv2d(_MaskedLayer):
     self._setup(name or 'Conv', (k, k, int(in_channels), int(units)), device, registry,
                 kernel_initializer)
     self.patch_mode = (int(in_channels) % 8 != 0) and k > 1
-    # small-Cin fast path (window tensor maps over a zero-bordered 8-channel copy of the input)
-    # (measured slower than the patch matrix for the ResNet stem at b256 -- its wgrad re-reads dY
-    # once per filter row -- so it is opt-in: layers.STEM_WINDOW_PATH = True)
-    self.smallc_mode = (STEM_WINDOW_PATH and self.patch_mode and int(in_channels) <= 8 and k <= 8 and
-                        int(units) % 8 == 0 and s in (1, 2))
     if self.patch_mode:
       self._kdim = k * k * int(in_channels)
       self._kpitch = (self._kdim + 7) // 8 * 8
       nbytes = int(_cabi.lib().rigl_packed_weights_bytes(1, self._kdim, self._cout))
       self.packed_patch = torch.zeros(nbytes, dtype=torch.uint8, device=device)
-    if self.smallc_mode:
-      self.packed_smallc = torch.zeros(k * int(units) * 64 * 2, dtype=torch.uint8, device=device)
-    self._use_smallc = False
     self.s2d_mode = bool(STEM_S2D_PATH and self.patch_mode and k == 7 and s == 2 and int(in_channels) <= 3 and
                          int(units) <= 64 and int(units) % 8 == 0 and padding == 'FIXED')
     if self.s2d_mode:
@@ -393,18 +384,12 @@ class SparseConv2d(_MaskedLayer):
       super(SparseConv2d, self).pack()
 
   def pack_special(self):
-    """The stem's own operand formats (space-to-depth / window kernels)."""
-    if self.patch_mode:
-      if self.s2d_mode:
-        d = self._desc(1, 16, 16)
-        _cabi.check(_cabi.lib().rigl_stem_s2d_pack_weights(
-            d, self.weight.data_ptr(), self.mask.bits.data_ptr(), self.packed_s2d.data_ptr(),
-            _cabi.stream_ptr()), 'rigl_stem_s2d_pack_weights')
-      if self.smallc_mode:
-        d = self._desc(1, max(self.ksize, 8), max(self.ksize, 8))
-        _cabi.check(_cabi.lib().rigl_smallc_pack_weights(
-            d, self.weight.data_ptr(), self.mask.bits.data_ptr(), self.packed_smallc.data_ptr(),
-            _cabi.stream_ptr()), 'rigl_smallc_pack_weights')
+    """The stem's own operand format (space-to-depth kernels)."""
+    if self.s2d_mode:
+      d = self._desc(1, 16, 16)
+      _cabi.check(_cabi.lib().rigl_stem_s2d_pack_weights(
+          d, self.weight.data_ptr(), self.mask.bits.data_ptr(), self.packed_s2d.data_ptr(),
+          _cabi.stream_ptr()), 'rigl_stem_s2d_pack_weights')
 
   @property
   def pad(self):
@@ -469,20 +454,6 @@ class SparseConv2d(_MaskedLayer):
                                                   _cabi.stream_ptr()), 'rigl_stem_s2d_fprop')
       self._patch_cache = xs
       return y
-    self._use_smallc = bool(self.smallc_mode and _cabi.lib().rigl_smallc_supported(d))
-    if self._use_smallc:
-      try:
-        xp = torch.empty(int(_cabi.lib().rigl_smallc_padded_bytes(d)), dtype=torch.uint8, device=x.device)
-        _cabi.check(_cabi.lib().rigl_smallc_pad_input(d, x.data_ptr(), xp.data_ptr(), _cabi.stream_ptr()),
-                    'rigl_smallc_pad_input')
-        _cabi.check(_cabi.lib().rigl_smallc_fprop(d, xp.data_ptr(), self.packed_smallc.data_ptr(), y.data_ptr(),
-                                                  _cabi.stream_ptr()), 'rigl_smallc_fprop')
-        self._patch_cache = xp
-        return y
-      except _cabi.RiglError as e:       # e.g. a driver that rejects the window tensor map
-        if 'cuTensorMapEncodeTiled' not in str(e):
-          raise
-        self.smallc_mode = self._use_smallc = False
     if self.patch_mode:
       self._patch_cache = src = self._patches(x)
       d, packed = self._patch_desc(src.shape[0]), self.packed_patch
@@ -526,13 +497,6 @@ class SparseConv2d(_MaskedLayer):
       _cabi.check(_cabi.lib().rigl_stem_s2d_wgrad(
           d, xs.data_ptr(), dy.data_ptr(), out.data_ptr(), 1.0 if accumulate else 0.0, ws.data_ptr(),
           ws.numel(), _cabi.stream_ptr()), 'rigl_stem_s2d_wgrad')
-      return
-    if self._use_smallc and getattr(self, '_patch_cache', None) is not None:
-      xp, self._patch_cache = self._patch_cache, None
-      ws = _workspace(x.device, _cabi.lib().rigl_smallc_workspace_bytes(d))
-      _cabi.check(_cabi.lib().rigl_smallc_wgrad(
-          d, xp.data_ptr(), dy.data_ptr(), out.data_ptr(), 1.0 if accumulate else 0.0, ws.data_ptr(),
-          ws.numel(), _cabi.stream_ptr()), 'rigl_smallc_wgrad')
       return
     if self.patch_mode:
       src = self._patch_cache if getattr(self, '_patch_cache', None) is not None else self._patches(x)

@@ -45,7 +45,7 @@ CONV_CASES = [
     (2, 9, 7, 8, 16, 3, 2, 0.8),
     (3, 8, 8, 64, 64, 1, 1, 0.0),
     (2, 14, 14, 64, 128, 1, 2, 0.4),
-    (2, 12, 12, 3, 8, 7, 2, 0.14),      # stem-like: cin=3 (small-Cin window-map path / SIMT)
+    (2, 12, 12, 3, 8, 7, 2, 0.14),      # stem-like: cin=3 (patch matrix / SIMT)
     (3, 32, 32, 3, 64, 7, 2, 0.14),
     (2, 17, 17, 3, 16, 3, 1, 0.3),
     (4, 16, 16, 64, 64, 3, 1, 0.64),
@@ -157,17 +157,6 @@ def test_rank_and_channel_errors():
     layer(torch.zeros(2, 4, 4, 4, device=DEV))
 
 
-@pytest.mark.parametrize('case', [(2, 12, 12, 3, 8, 7, 2, 0.14), (3, 32, 32, 3, 64, 7, 2, 0.14), (2, 17, 17, 3, 16, 3, 1, 0.3)])
-def test_conv_stem_window_path(case):
-  """The opt-in small-Cin path (zero-bordered 8-channel input + overlapping-window tensor maps)."""
-  from rigl_b200 import layers
-  layers.STEM_WINDOW_PATH = True
-  try:
-    _conv_case(case, force_simt=False)
-  finally:
-    layers.STEM_WINDOW_PATH = False
-
-
 @pytest.mark.parametrize('case', [(2, 16, 16, 3, 64, 7, 2, 0.14), (3, 32, 32, 3, 64, 7, 2, 0.14),
                                   (2, 64, 48, 3, 16, 7, 2, 0.5), (2, 224, 224, 3, 64, 7, 2, 0.14)])
 def test_conv_stem_s2d_path(case):
@@ -180,7 +169,8 @@ def test_conv_stem_s2d_path(case):
     layers.STEM_S2D_PATH = old
 
 
-@pytest.mark.parametrize('case', [(3, 32, 32, 3, 64, 7, 2, 0.14), (2, 64, 48, 3, 16, 7, 2, 0.5)])
+@pytest.mark.parametrize('case', [(3, 32, 32, 3, 64, 7, 2, 0.14), (2, 64, 48, 3, 16, 7, 2, 0.5),
+                                  (2, 12, 12, 3, 8, 7, 2, 0.14), (2, 17, 17, 3, 16, 3, 1, 0.3)])
 def test_conv_stem_patch_matrix_path(case):
   """RIGL_STEM_S2D=0 fallback: the im2col patch-matrix stem."""
   from rigl_b200 import layers
@@ -189,18 +179,6 @@ def test_conv_stem_patch_matrix_path(case):
     _conv_case(case, force_simt=False)
   finally:
     layers.STEM_S2D_PATH = old
-
-
-@pytest.mark.parametrize('case', [CONV_CASES[5], CONV_CASES[8], CONV_CASES[10], CONV_CASES[11]])
-def test_conv_cluster_multicast_path(case):
-  """Same results with the 2-CTA multicast clusters (run in a subprocess: the switch is read once)."""
-  import os, subprocess, sys
-  code = ('import sys; sys.path.insert(0, %r); sys.path.insert(0, %r); import test_conv_gpu as t; '
-          't._conv_case(%r, False); print("MC_OK")' % (os.path.dirname(os.path.dirname(__file__)),
-                                                       os.path.dirname(__file__), case))
-  env = dict(os.environ, RIGL_CLUSTER_MC='1', RIGL_CTA_PAIR='0')
-  out = subprocess.run([sys.executable, '-c', code], env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
-  assert 'MC_OK' in out.stdout, out.stdout[-1500:]
 
 
 # 3x3 / stride 1 / pad 1 layers with <= 64 reduction channels run on the halo kernels (one halo tile in
@@ -233,7 +211,8 @@ def test_conv_halo_disabled_matches(case):
   assert 'GEN_OK' in out.stdout, out.stdout[-1500:]
 
 
-@pytest.mark.parametrize('case', [CONV_CASES[0], CONV_CASES[5], CONV_CASES[7], CONV_CASES[9], CONV_CASES[12]])
+@pytest.mark.parametrize('case', [CONV_CASES[0], CONV_CASES[5], CONV_CASES[7], CONV_CASES[8], CONV_CASES[9], CONV_CASES[10],
+                                  CONV_CASES[11], CONV_CASES[12]])
 def test_conv_single_cta_mma_path(case):
   """The default K-major kernel is the CTA-pair one (cta_group::2); this keeps the single-CTA
   (M = 128) kernel covered."""
@@ -356,23 +335,9 @@ def test_batched_pack_equals_per_layer_pack():
   layers._PACKED_AHEAD.clear()
 
 
-@pytest.mark.parametrize('case', [CONV_CASES[8], CONV_CASES[9], CONV_CASES[11]])
-def test_conv_wgrad_in_kernel_splitk_fixup_path(case):
-  """RIGL_WGRAD_FIXUP=1 (opt-in; measured slower on the BASELINE shapes): the dense wgrad's split-K partials are
-  summed by the last-arriving CTA inside the wgrad kernel instead of by a separate k_splitk_reduce launch.  Same
-  oracle, same tolerance."""
-  import os, subprocess, sys
-  code = ('import sys; sys.path.insert(0, %r); sys.path.insert(0, %r); import test_conv_gpu as t; '
-          't._conv_case(%r, False); print("RED_OK")' % (os.path.dirname(os.path.dirname(__file__)),
-                                                        os.path.dirname(__file__), case))
-  env = dict(os.environ, RIGL_WGRAD_FIXUP='1')
-  out = subprocess.run([sys.executable, '-c', code], env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
-  assert 'RED_OK' in out.stdout, out.stdout[-1500:]
-
-
 def test_conv_wgrad_accumulates_over_backward_passes():
-  """beta = 1: a second backward before the gradients are consumed ADDS to the dense gradient (the in-kernel
-  split-K fix-up reads dw back and adds the partials to it in split order)."""
+  """beta = 1: a second backward before the gradients are consumed ADDS to the dense gradient (k_splitk_reduce
+  reads dw back and adds the split-K partials to it in split order)."""
   pruning.reset_default_registry()
   torch.manual_seed(3)
   layer = SparseConv2d(128, 256, 3, padding='FIXED', name='acc', device=DEV)

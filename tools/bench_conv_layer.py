@@ -1,7 +1,7 @@
 """Per-layer micro-benchmark of the masked conv kernels (fprop / dgrad / dense wgrad) through the
 same host calls the training step makes.  One JSON line per (shape, op): microseconds (CUDA
 events, median of --iters, inputs rotated through buffers larger than L2), dense-executed TFLOP/s
-and algorithmic GB/s.  Kernel-selection switches (RIGL_HALO3X3, RIGL_HALO_CFG, RIGL_CTA_PAIR ...)
+and algorithmic GB/s.  Kernel-selection switches (RIGL_HALO3X3, RIGL_CTA_PAIR, RIGL_TMA_STORE ...)
 are read once per process: run one process per configuration.
 
   python tools/bench_conv_layer.py [--shapes r50s1] [--iters 20] [--tag name]
@@ -82,7 +82,7 @@ def main():
         return layer._fprop(xs[i % copies], None, False)
       finally:
         L.FUSE_BN_STATS, layer.collect_bn_stats = False, False
-    _cabi.lib().rigl_set_bn_stats_always(1 | (int(os.environ.get('STATS_DBG', '0')) << 4))
+    _cabi.lib().rigl_set_bn_stats_always(1)
     L.FUSE_BN_STATS = False
     ops = (('fprop', lambda i: layer._fprop(xs[i % copies], None, False)), ('fprop_stats', fprop_stats),
            ('dgrad', lambda i: layer._dgrad(dys[i % copies], xs[i % copies])),

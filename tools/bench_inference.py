@@ -92,7 +92,7 @@ def timed(fn, seconds):
 
 
 def kind_of(name):
-  if any(k in name for k in ('k_igemm', 'k_halo3x3', 'k_stem_s2d', 'k_simt_fprop', 'k_smallc', 'k_im2col')):
+  if any(k in name for k in ('k_igemm', 'k_halo3x3', 'k_stem_s2d', 'k_simt_fprop', 'k_im2col')):
     return 'fprop'
   if 'k_bn_' in name:
     return 'bn'

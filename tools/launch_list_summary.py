@@ -10,7 +10,7 @@ import re
 import sys
 
 FAMILIES = [
-    ('conv', r'k_igemm|k_halo3x3|k_stem_s2d|k_splitk|k_im2col|k_simt|k_smallc|k_pack_weights|k_s2d'),
+    ('conv', r'k_igemm|k_halo3x3|k_stem_s2d|k_splitk|k_im2col|k_simt|k_pack_weights|k_s2d'),
     ('bn', r'k_bn_'),
     ('pool', r'k_maxpool'),
     ('optimizer', r'k_sgd|multi_tensor_apply'),
